@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- audio-hours/sec of the inaSpeechSegmenter hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One step = one pass of the whole hot path (K1 log-mel/energy -> energy Viterbi
 -> smn CNN -> Viterbi -> gender CNN -> Viterbi -> segment list on the host) over
@@ -27,6 +27,10 @@ The same JSON line carries, all measured in this run and outside the timed regio
 restatement + C Viterbi: TensorFlow and the .hdf5 networks are not installable here) the way the
 reference scales out (one worker process per file chunk, scripts/ina_speech_segmenter_pyro_client.py:64-74):
 host_cores/16 workers x 16 threads on disjoint 10-minute chunks.
+
+`--dump-outputs DIR` writes the segment list the last timed step returned (b200 arm, rank 0) to
+DIR/segments.npy: float64 [n, 3], one row (index into SEGMENT_LABELS, start s, stop s) per segment.
+The synthetic input is seeded, so two builds run with the same arguments can be compared row for row.
 """
 import argparse
 import json
@@ -44,12 +48,20 @@ sys.path.insert(0, ROOT)
 METRIC = 'audio-hours/sec segmented (16 kHz mono)'
 UNIT = 'audio-hours/s'
 SR = 16000
+SEGMENT_LABELS = ('noEnergy', 'energy', 'speech', 'music', 'noise', 'female', 'male')
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError('must be at least 1, got %d' % v)
+    return v
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=3)
+    ap.add_argument('--steps', type=positive_int, default=3, help='timed steps')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--hours', type=float, default=10.0, help='audio hours per GPU per step')
@@ -63,7 +75,18 @@ def parse():
     ap.add_argument('--k1-hours', type=float, default=100.0, help='BASELINE configs[2] size')
     ap.add_argument('--vbx-hours', type=float, default=50.0, help='BASELINE configs[3] size (1 h files)')
     ap.add_argument('--vbx-max-sec', type=float, default=60.0, help='stop the VBx leg after this many seconds (bounded sample)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the segment list of the last timed step to DIR/segments.npy')
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
+    return args
+
+
+def dump_outputs(out_dir, segs):
+    """[(label, start s, stop s)] -> DIR/segments.npy, float64 [n, 3] (label as its index in SEGMENT_LABELS)."""
+    rows = np.array([(SEGMENT_LABELS.index(lab), a, b) for lab, a, b in segs], dtype=np.float64).reshape(-1, 3)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'segments.npy'), rows)
 
 
 # ----------------------------------------------------------------------------- synthetic audio
@@ -668,6 +691,8 @@ def run_b200(args):
         if world > 1:
             dist.destroy_process_group()
         return 0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, segs)
 
     peaks = {}
     try:

@@ -189,6 +189,24 @@ def test_bench_reference_arm_contract():
     assert d['e2e']['h2d_bytes_per_step'] == 0 and d['e2e']['value'] == d['value']
 
 
+def test_bench_dump_outputs_and_argument_checks(tmp_path):
+    """`bench.py --dump-outputs DIR` stores the segment list losslessly as float64 (label code, start, stop) rows;
+    a run without timed steps, or a dump from the CPU arm, is refused before anything runs."""
+    import subprocess
+    import sys
+    import bench
+    segs = [('noEnergy', 0.0, 1.98), ('female', 1.98, 3.5), ('music', 3.5, 29.080000000000002), ('noise', 29.080000000000002, 30.0)]
+    bench.dump_outputs(str(tmp_path / 'out'), segs)
+    got = np.load(tmp_path / 'out' / 'segments.npy')
+    assert got.dtype == np.float64 and got.shape == (4, 3)
+    assert [(bench.SEGMENT_LABELS[int(c)], a, b) for c, a, b in got] == segs
+    for extra in (['--steps', '0'], ['--impl', 'reference', '--dump-outputs', str(tmp_path / 'ref')]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py')] + extra, stdout=subprocess.PIPE,
+                             stderr=subprocess.PIPE, text=True, timeout=120)
+        assert out.returncode == 2 and 'usage:' in out.stderr, extra
+    assert not (tmp_path / 'ref').exists()
+
+
 def test_ffmpeg_branch_with_stand_in_binary(media, tmp_path):
     """The ffmpeg subprocess branch of media2sig16kmono (reference io.py:60-79): no ffmpeg exists in any of the
     boxes, so a stand-in executable checks the argv the reference builds (-i <media> -f wav -acodec pcm_s16le
